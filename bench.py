@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's B200 kernel path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU trainer path (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed step's results to DIR/*.npy
 
 One "step" = one full pass of the hot path over one batch: zero_grad -> forward -> CE loss -> backward ->
 (all-reduce) -> fused SGD step, batch 256 per GPU, bf16 compute / fp32 masters.  Prints ONE JSON line
@@ -44,7 +45,30 @@ def parse():
     p.add_argument('--no-e2e', action='store_true')
     p.add_argument('--no-cpu-baseline', action='store_true')
     p.add_argument('--cpu-batch', type=int, default=32)
-    return p.parse_args()
+    p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                   help='after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32): '
+                        'logits, loss, the updated parameters and the BatchNorm running statistics (a fixed sample of '
+                        'an array larger than 16 MB)')
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error('--steps must be at least 1 (the number of timed steps)')
+    return args
+
+
+DUMP_MAX_ELEMS = 1 << 22   # per array: 16 MB of float32, so that the four arrays of a dump stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor as path/<name>.npy in float32.  A tensor larger than DUMP_MAX_ELEMS is replaced by a fixed
+    sample of its flattened elements (seed 0, ascending index order), identical from run to run for the same shape."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.flatten()[idx.to(t.device)]
+        np.save(os.path.join(path, name + '.npy'), t.cpu().numpy())
 
 
 def peaks():
@@ -210,12 +234,12 @@ def main():
             loss = criterion(out, y_dev)
             loss.backward()
         else:
-            loss = replayed[1]
+            out, loss = replayed[0], replayed[1]
         trainer._allreduce_gradients()
         optimizer.set_grad_unscale(1.0, world)
         optimizer.step()
         trainer.training_steps += 1
-        return loss
+        return out, loss
 
     for _ in range(max(args.warmup, 4)):   # steps 1-2 eager, 3 captures the CUDA graph, 4+ replay it
         device_step()
@@ -228,7 +252,7 @@ def main():
     e0.record()
     t_enq = time.perf_counter()
     for _ in range(args.steps):
-        loss = device_step()
+        out, loss = device_step()
     e1.record()
     enqueue_ms = (time.perf_counter() - t_enq) * 1e3 / args.steps     # host time to launch one step (no syncs)
     torch.cuda.synchronize()
@@ -240,6 +264,13 @@ def main():
     ms = float(t)
     clocks = sampler.stop() if sampler else None
     final_loss = float(loss.detach())
+    if args.dump_outputs and rank == 0:
+        # before the e2e windows below train the model further
+        dump_outputs(args.dump_outputs, {
+            'logits': out, 'loss': loss.reshape(1),
+            'params': torch.cat([p.detach().flatten() for p in model.parameters()]),
+            'bn_running_stats': torch.cat([b.detach().float().flatten() for n, b in model.named_buffers()
+                                           if 'running' in n])})
     sync_all()
 
     # ---- end to end through the public API: pinned host batches, H2D + loss D2H inside the timed region ----

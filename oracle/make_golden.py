@@ -1,8 +1,9 @@
-"""Generates tests/golden/* by running the UNMODIFIED reference (read-only at /root/reference) in this
-container.  Run once from the repo root:  python oracle/make_golden.py
+"""Generates tests/golden/* by running the UNMODIFIED reference (a checkout of eladhoffer/convNet.pytorch, named by
+the environment variable B200_REFERENCE).  Run from the repo root:  B200_REFERENCE=<checkout> python oracle/make_golden.py
 The fixtures pin (a) the oracle restatement (oracle/ref_model.py), (b) the re-authored host code
 (models, regimes, trainer) and (c) -- through the GPU tests -- the CUDA pipeline.
-Nothing here is needed at test time: tests read only the committed fixtures.
+The reference is not needed at test time: tests read only the committed fixtures, in the encodings of
+oracle/fixtures.py.
 """
 import json
 import os
@@ -12,11 +13,18 @@ from copy import deepcopy
 import numpy as np
 import torch
 
-REF = os.environ.get('B200_REFERENCE', '/root/reference')
-OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'tests', 'golden')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+from oracle.fixtures import bf16_bits, synth_record, synthetic_momentum  # noqa: E402
+
+REF = os.environ.get('B200_REFERENCE')
+OUT = os.path.join(ROOT, 'tests', 'golden')
 
 
 def import_reference():
+    if not REF:
+        raise SystemExit('make_golden.py: set B200_REFERENCE to a checkout of the reference')
     sys.path.insert(0, REF)
     import models as ref_models            # noqa: E402
     import trainer as ref_trainer          # noqa: E402
@@ -34,9 +42,11 @@ def tensor_stats(sd):
     return out
 
 
-def synth(batch, shape, classes, seed=0):
-    g = torch.Generator().manual_seed(seed)
-    return torch.randn(batch, *shape, generator=g), torch.randint(0, classes, (batch,), generator=g)
+SAMPLE = 256   # elements per tensor kept of gradients and updated parameters
+
+
+def sample_index(numel, rng):
+    return np.arange(numel) if numel <= SAMPLE else np.sort(rng.choice(numel, SAMPLE, replace=False))
 
 
 def mobilenet_v2_fixture(ref_models, ref_trainer, ref_optim, ref_ce):
@@ -48,7 +58,7 @@ def mobilenet_v2_fixture(ref_models, ref_trainer, ref_optim, ref_ce):
     seed (test_model_factories_match_reference_init pins that)."""
     torch.manual_seed(123)
     model = ref_models.mobilenet_v2(dataset='imagenet')
-    x, y = synth(16, (3, 96, 96), 1000)
+    x, y, rec = synth_record(16, (3, 96, 96), 1000)
     opt = ref_optim.OptimRegime(model, model.regime)
     tr = ref_trainer.Trainer(model, ref_ce.CrossEntropyLoss(), opt, device_ids=None, device='cpu',
                              dtype=torch.float, print_freq=1000)
@@ -64,7 +74,7 @@ def mobilenet_v2_fixture(ref_models, ref_trainer, ref_optim, ref_ce):
     post = tensor_stats(model.state_dict())
     torch.manual_seed(1001)
     _, loss2, _ = tr._step(x, y, training=True)
-    np.savez(os.path.join(OUT, 'mobilenet_v2_summary.npz'), x=x.numpy(), y=y.numpy(), logits=out.detach().numpy(),
+    np.savez(os.path.join(OUT, 'mobilenet_v2_summary.npz'), **rec, logits=out.detach().numpy(),
              loss=np.float64(float(loss)), loss_step2=np.float64(float(loss2)), grad_names=np.array(list(gn.keys())),
              grad_norms=np.array(list(gn.values())), grad_heads=np.stack([gh[n] for n in gn]),
              wd_names=np.array(wd_names), post_names=np.array(list(post.keys())),
@@ -89,8 +99,8 @@ def neighbours_fixture(ref_models, ref_ce):
     networks carry 1e-3 of rounding noise in the SE variants) -- logits, loss, every parameter-gradient norm,
     running-statistics sums.  Pins oracle.ref_model's restatement of those families (tests/test_oracle_golden.py)."""
     blob = {}
-    x, y = synth(8, (3, 96, 96), 1000, seed=7)
-    blob['x'], blob['y'] = x.numpy(), y.numpy()
+    x, y, rec = synth_record(8, (3, 96, 96), 1000, seed=7)
+    blob.update(rec)
     crit = ref_ce.CrossEntropyLoss()
     for name, factory, cfg in NEIGHBOURS:
         torch.manual_seed(123)
@@ -103,7 +113,7 @@ def neighbours_fixture(ref_models, ref_ce):
         with torch.no_grad():
             for n, p in model.named_parameters():
                 if p.dim() == 1 and ('bn' in n or n.split('.')[-2].isdigit() or 'downsample' in n) and n.endswith('weight'):
-                    p.copy_(0.5 + torch.rand(p.shape, generator=g))
+                    p.copy_((0.5 + torch.rand(p.shape, generator=g)).to(torch.bfloat16).float())
         init = {k: v.clone() for k, v in model.state_dict().items()}
         model.double()                  # fp64: the comparison with the restatement is then free of rounding noise
         model.train()
@@ -125,7 +135,7 @@ def neighbours_fixture(ref_models, ref_ce):
         # the perturbed affine parameters (everything else is re-created from the seed by the test)
         for k, v in init.items():
             if v.dim() == 1 and v.is_floating_point() and 'running' not in k and k.endswith('weight'):
-                blob[name + '/affine/' + k] = v.numpy()
+                blob[name + '/affine/' + k] = bf16_bits(v)
         print(name, 'loss %.5f' % float(loss), '%d gradients' % len(names))
     np.savez_compressed(os.path.join(OUT, 'neighbours.npz'), **blob)
     print('neighbours fixture written')
@@ -165,7 +175,7 @@ def main():
     # ---- 2. resnet20: reference Trainer + OptimRegime, 5 warm-up steps then one recorded step ----
     torch.manual_seed(123)
     model = ref_models.resnet(dataset='cifar10', depth=20)
-    x, y = synth(8, (3, 32, 32), 10)
+    x, y, rec = synth_record(8, (3, 32, 32), 10)
     crit = ref_ce.CrossEntropyLoss()
     opt = ref_optim.OptimRegime(model, model.regime)
     tr = ref_trainer.Trainer(model, crit, opt, device_ids=None, device='cpu', dtype=torch.float, print_freq=1000)
@@ -174,8 +184,15 @@ def main():
     for _ in range(5):
         _, loss, _ = tr._step(x, y, training=True)
         losses.append(float(loss))
+    # the recorded step starts from this state with its parameters rounded to bf16, which the fixture then holds exactly
+    # in half the bytes (the running statistics stay fp32), and from seeded momentum buffers
+    mom_seed = 5
+    mom_b = synthetic_momentum([(n, p.shape) for n, p in model.named_parameters()], mom_seed)
+    with torch.no_grad():
+        for n, p in model.named_parameters():
+            p.copy_(p.to(torch.bfloat16).float())
+            opt.optimizer.state[p]['momentum_buffer'].copy_(mom_b[n])
     state_b = deepcopy(model.state_dict())
-    mom_b = {n: opt.optimizer.state[p]['momentum_buffer'].clone() for n, p in model.named_parameters()}
     # recorded step: capture grads before the optimizer touches them
     opt.zero_grad(); opt.update(0, tr.training_steps)
     out = model(x); loss = crit(out, y); loss.backward()
@@ -184,17 +201,21 @@ def main():
         p.grad.data.div_(1.0)
     opt.step()
     post = deepcopy(model.state_dict())
-    blob = {'x': x.numpy(), 'y': y.numpy(), 'logits': out.detach().numpy(), 'loss': np.float64(float(loss)),
-            'warm_losses': np.array(losses)}
+    blob = {**rec, 'logits': out.detach().numpy(), 'loss': np.float64(float(loss)), 'warm_losses': np.array(losses),
+            'mom_seed': np.int64(mom_seed), 'mom_names': np.array([n for n, _ in model.named_parameters()])}
     for k, v in state_b.items():
-        blob['state/' + k] = v.numpy()
-    for k, v in mom_b.items():
-        blob['mom/' + k] = v.numpy()
+        blob['state/' + k] = bf16_bits(v) if k in grads else v.numpy()
+    # per parameter: the norm of its gradient, and the gradient and updated value at a fixed sample of elements
+    rng = np.random.default_rng(0)
     for k, v in grads.items():
-        blob['grad/' + k] = v.numpy()
+        idx = sample_index(v.numel(), rng)
+        blob['idx/' + k] = idx
+        blob['grad_norm/' + k] = np.float64(v.double().norm())
+        blob['grad/' + k] = v.flatten().numpy()[idx]
+        blob['post_norm/' + k] = np.float64(post[k].double().norm())
     for k, v in post.items():
-        blob['post/' + k] = v.numpy()
-    np.savez(os.path.join(OUT, 'resnet20_step.npz'), **blob)
+        blob['post/' + k] = v.flatten().numpy()[blob['idx/' + k]] if k in grads else v.numpy()
+    np.savez_compressed(os.path.join(OUT, 'resnet20_step.npz'), **blob)
 
     # ---- 3. reference Trainer.train loop over a tiny loader (loop-level golden) ----
     torch.manual_seed(123)
@@ -214,7 +235,7 @@ def main():
     # ---- 4. resnet50 summary at a small size: 2 warm steps then a recorded step ----
     torch.manual_seed(123)
     model = ref_models.resnet(dataset='imagenet', depth=50)
-    x50, y50 = synth(4, (3, 64, 64), 1000)
+    x50, y50, rec50 = synth_record(4, (3, 64, 64), 1000)
     opt = ref_optim.OptimRegime(model, model.regime)
     tr = ref_trainer.Trainer(model, ref_ce.CrossEntropyLoss(smooth_eps=0.1), opt, device_ids=None, device='cpu',
                              dtype=torch.float, print_freq=1000)
@@ -226,7 +247,7 @@ def main():
     opt.zero_grad()
     out = model(x50); loss = tr.criterion(out, y50); loss.backward()
     gn = {n: float(p.grad.norm()) for n, p in model.named_parameters()}
-    np.savez(os.path.join(OUT, 'resnet50_summary.npz'), x=x50.numpy(), y=y50.numpy(), logits=out.detach().numpy(),
+    np.savez(os.path.join(OUT, 'resnet50_summary.npz'), **rec50, logits=out.detach().numpy(),
              loss=np.float64(float(loss)), warm_losses=np.array(l50),
              grad_names=np.array(list(gn.keys())), grad_norms=np.array(list(gn.values())))
 

@@ -202,10 +202,11 @@ def test_evaluate_cli_cpu(tmp_path):
     assert both['loss'] > 0 and 0 <= both['prec1'] <= 100
 
 
-def test_committed_profile_feeds_bench_traffic():
+def test_committed_profile_feeds_bench_traffic(tmp_path):
     """bench.py reports roofline.traffic from profiles/r02_traffic.json (DRAM bytes per launch of the dominant kernel
-    class, produced by tools/summarize_launches.py from the committed ncu launch list): the file must carry the class
-    bench.py looks up, and the summariser must reproduce it from the committed CSV."""
+    class, produced by tools/summarize_launches.py from the committed ncu launch list profiles/r02_launches.csv): the
+    file must carry the class bench.py looks up, and the summariser must reproduce it from that launch list, stored
+    gzip-compressed as tests/golden/r02_launches.csv.gz."""
     import json
     import subprocess
     import sys
@@ -214,9 +215,9 @@ def test_committed_profile_feeds_bench_traffic():
         tj = json.load(f)['classes']
     for key in ('conv_fprop+dgrad', 'conv_wgrad', 'bn_apply', 'bn_bwd_dx', 'bn_bwd_reduce'):
         assert tj[key]['launches'] > 0 and tj[key]['dram_read_bytes'] > 0, key
-    out_md, out_js = os.path.join('/tmp', 'r02_launches_check.md'), os.path.join('/tmp', 'r02_traffic_check.json')
+    out_md, out_js = str(tmp_path / 'r02_launches_check.md'), str(tmp_path / 'r02_traffic_check.json')
     r = subprocess.run([sys.executable, os.path.join(root, 'tools', 'summarize_launches.py'),
-                        os.path.join(root, 'profiles', 'r02_launches.csv'), out_md, 'check', out_js],
+                        os.path.join(root, 'tests', 'golden', 'r02_launches.csv.gz'), out_md, 'check', out_js],
                        capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stderr[-500:]
     with open(out_js) as f:

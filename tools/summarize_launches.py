@@ -1,11 +1,19 @@
 """Summarise an ncu launch list (`--metrics gpu__time_duration.sum[,dram__bytes_read.sum,dram__bytes_write.sum] --csv`):
 per-kernel totals of ONE training step (the launches between the last two fused_sgd kernels) -> markdown, plus a JSON with
 the DRAM traffic per bench.py kernel class (`roofline.traffic`).
-usage: summarize_launches.py in.csv out.md [title] [out.json]"""
+usage: summarize_launches.py in.csv[.gz] out.md [title] [out.json]
+A launch list named *.gz is read gzip-compressed (the test input tests/golden/r02_launches.csv.gz is the compressed
+profiles/r02_launches.csv)."""
 import collections
 import csv
+import gzip
 import json
 import sys
+
+
+def open_text(path):
+    return gzip.open(path, 'rt') if path.endswith('.gz') else open(path)
+
 
 CLASSES = {   # kernel-name prefix -> class name used by bench.py (ops._T)
     'conv_wgrad': 'conv_wgrad', 'conv_halo_wgrad': 'conv_wgrad',
@@ -16,7 +24,7 @@ CLASSES = {   # kernel-name prefix -> class name used by bench.py (ops._T)
 
 
 def main(src, dst, title, js=None):
-    with open(src) as f:
+    with open_text(src) as f:
         lines = [l for l in f if l.startswith('"')]
     r = csv.reader(lines)
     hdr = next(r)
